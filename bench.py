@@ -34,6 +34,13 @@ SECONDARY (same line):
 
 `--impl reference`: the reference's CPU search on all host threads as its own arm; each step is a bounded sample of
 the workload (the whole N=16 / 15 / 14 search, by core count: the same code per node, 1/7 .. 1/300 of the tree).
+
+`--dump-outputs DIR`: after the headline's timed steps, what its last step returned, so that two builds can be
+compared output for output (the inputs are the same every run: the warm-up pool of step 1 is deterministic):
+  step2_pools    float64 [pools, 5] of the resident-pool offload loop (1 GPU): per device pool the rounds, parents
+                 popped, children pushed and solutions that tsb_nq_pool_run_multi returned over the step, and the
+                 nodes left in the pool when all pools held fewer than m
+  search_counts  float64 [explored tree, solutions] of the last whole search (the only file with N > 1)
 """
 import argparse
 import json
@@ -329,8 +336,8 @@ def run_headline_1gpu(steps, warmup, device_index, M=M_HEAD, N=N_HEAD):
 
     def step2():
         """the driver's step 2 on resident pools (nq_devpool_multi_rounds): shared launches, dry pools take the oldest
-        half of the fullest one; -> (rounds, children, solutions)"""
-        tot = [0, 0, 0]
+        half of the fullest one; -> [rounds, parents, children, solutions] per pool"""
+        per = [[0, 0, 0, 0] for _ in evs]
         while True:
             sizes = [e.pool_size for e in evs]
             for i, e in enumerate(evs):
@@ -340,9 +347,9 @@ def run_headline_1gpu(steps, warmup, device_index, M=M_HEAD, N=N_HEAD):
                         e.pool_steal_from(evs[v], m_HEAD)
                         sizes = [x.pool_size for x in evs]
             if max(sizes) < m_HEAD:
-                return tot
-            for nr, _np, nc, ns in tsb200.nqueens_pool_run_multi(evs, m_HEAD, M, 2048):
-                tot = [tot[0] + nr, tot[1] + nc, tot[2] + ns]
+                return per
+            for i, r in enumerate(tsb200.nqueens_pool_run_multi(evs, m_HEAD, M, 2048)):
+                per[i] = [a + b for a, b in zip(per[i], r)]
 
     stream = torch.cuda.ExternalStream(ev.stream, device=dev)
     want = GOLDEN_NQ[N]
@@ -364,15 +371,16 @@ def run_headline_1gpu(steps, warmup, device_index, M=M_HEAD, N=N_HEAD):
             # (every launch inside is followed by a stream synchronisation, so the two events bracket all of it
             # whichever pool's stream a launch went to)
             e0.record(stream)
-            nr, nc, ns = step2()
+            per = step2()
             e1.record(stream)
             torch.cuda.synchronize()
             t_dev += e0.elapsed_time(e1) / 1e3
+            nr, _, nc, ns = (sum(p[k] for p in per) for k in range(4))
             nodes += nc
             rounds += nr
             launches_per_step = n_launches() - launches_before
-            left = sum(e.pool_drain().shape[0] for e in evs)
-            assert wtree + nc + left <= want[0] and ns + wsol <= want[1]
+            left = [e.pool_drain().shape[0] for e in evs]
+            assert wtree + nc + sum(left) <= want[0] and ns + wsol <= want[1]
         launches = n_launches() - l0
         # ---- e2e: the whole search, host in / host out
         torch.cuda.synchronize()
@@ -386,9 +394,12 @@ def run_headline_1gpu(steps, warmup, device_index, M=M_HEAD, N=N_HEAD):
         t_e2e = time.perf_counter() - t0
     for e in evs:
         e.close()
+    outputs = {"step2_pools": np.array([p + [n] for p, n in zip(per, left)], dtype=np.float64),
+               "search_counts": np.array([st.explored_tree, st.explored_sol], dtype=np.float64)}
     return {"pools": P, "t_dev": t_dev, "nodes": nodes, "rounds": rounds, "t_e2e": t_e2e, "tree": tree, "launches": launches,
             "launches_per_step": launches_per_step, "clocks": clk.summary(), "create_ms": t_create * 1e3,
-            "h2d": warm.nbytes, "d2h": 64 + P * m_HEAD * 21, "offloads": int(st.offloads), "steps": steps}
+            "h2d": warm.nbytes, "d2h": 64 + P * m_HEAD * 21, "offloads": int(st.offloads), "steps": steps,
+            "outputs": outputs}
 
 
 def run_headline_multi(steps, warmup, world, rank, M=M_HEAD, N=N_HEAD):
@@ -424,7 +435,8 @@ def run_headline_multi(steps, warmup, world, rank, M=M_HEAD, N=N_HEAD):
                "launches_per_step": launches // steps, "rounds": int(st.offloads) * steps, "offloads": int(st.offloads),
                "steps": steps, "h2d": 21 * m_HEAD * 4 * world, "d2h": (64 + 21 * m_HEAD * 4) * world, "steals": steals / steps,
                "pools": 4,
-               "per_gpu_share": shares, "create_ms": None}
+               "per_gpu_share": shares, "create_ms": None,
+               "outputs": {"search_counts": np.array([st.explored_tree, st.explored_sol], dtype=np.float64)}}
     dist_barrier(world, cpu=True)
     return out
 
@@ -593,6 +605,14 @@ def cpu_baseline_search(cores):
             "value_1core": t1 / dt1 / 1e6, "sample_1core": f"whole N=13 search, one thread ({dt1:.2f} s)"}
 
 
+def write_outputs(path, arrays):
+    """--dump-outputs: DIR/<name>.npy per array (float32 / float64; the headline's outputs are a few KB)"""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def emit(line):
     """print THE one JSON line on the real stdout (fd 1 is pointed at stderr while the bench runs, so that
     libraries that write to stdout on their own — NCCL prints its version there — cannot pollute it)"""
@@ -617,6 +637,8 @@ def main():
     ap.add_argument("--no-batch", action="store_true", help="skip the batch-evaluator legs")
     ap.add_argument("--no-search", action="store_true", help="skip the secondary whole searches")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline's last step returned as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank, local_rank, world = dist_env()
@@ -669,6 +691,8 @@ def main():
     else:
         h = run_headline_multi(args.steps, args.warmup, world, rank)
     line = None
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, h["outputs"])
     if rank == 0:
         value = h["nodes"] / h["t_dev"] / 1e6
         e2e = h["tree"] / h["t_e2e"] / 1e6

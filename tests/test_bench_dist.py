@@ -1,5 +1,6 @@
 """CPU checks of bench.py: the multi-rank reduction used for N > 1 (world_size-2 gloo run: max over ranks
-of the time, sum over ranks of the units — no collective in the data path) and the synthetic workloads."""
+of the time, sum over ranks of the units — no collective in the data path) and the synthetic workloads; on a GPU,
+the outputs --dump-outputs writes."""
 import json
 import os
 import socket
@@ -7,6 +8,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 import bench
 import tsb200
@@ -77,3 +79,32 @@ def test_synthetic_pfsp_parents():
     p = bench.synth_pfsp_parents(2048, 3, tsb200.PFSP_NODE_DTYPE)
     assert (p["limit1"] == p["depth"] - 1).all() and p["depth"].min() >= 1 and p["depth"].max() <= 19
     assert (np.sort(p["prmu"], axis=1) == np.arange(20)).all()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_headline_step(tmp_path):
+    """--dump-outputs writes float32 / float64 arrays of the last timed step, and they are what that step computed:
+    every node pushed (warm-up pool + children) was popped or left over, and with nothing left over, warm-up + step-2
+    children and solutions = the reference's N=17 counts"""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "0", "--no-batch",
+                        "--no-search", "--no-cpu", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout)["steps"] == 1
+    files = sorted(tmp_path.glob("*.npy"))
+    assert sum(f.stat().st_size for f in files) <= 64 << 20
+    out = {f.stem: np.load(f) for f in files}
+    assert set(out) == {"step2_pools", "search_counts"}
+    assert all(a.dtype in (np.float32, np.float64) and a.size for a in out.values())
+    want = bench.GOLDEN_NQ[17]
+    assert tuple(out["search_counts"]) == want
+    pools = out["step2_pools"].astype(np.int64)
+    assert pools.ndim == 2 and pools.shape[1] == 5 and (pools[:, 0] > 0).all()
+    _, parents, children, solutions, left = pools.sum(axis=0)
+    assert (pools[:, 4] < bench.m_HEAD).all()
+    warm, wtree, wsol = tsb200.nqueens_warmup(17, pools.shape[0] * bench.m_HEAD)
+    assert warm.shape[0] + children == parents + left  # steals move nodes between pools, none is lost
+    if left == 0:  # every pool ran dry: the search has nothing left for step 3
+        assert (wtree + children, wsol + solutions) == want
+    else:
+        assert wtree + children < want[0] and wsol + solutions <= want[1]
