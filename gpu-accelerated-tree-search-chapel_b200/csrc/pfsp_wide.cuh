@@ -47,6 +47,105 @@ struct PfspWideSmem {
   int32_t fc[PW_MAXM * PW_THREADS];  // lb2: the child's front, [machine][thread] (dynamically indexed by pair)
 };
 
+// Bounds of the children of one parent — the per-parent part of evaluate_gpu_lb1 / _lb1_d / _lb2: the parent's
+// front / remain (and, for lb2, its scheduled set) once, then emit(k, lb) for every slot k = limit1+1 .. jobs-1 in
+// order, lb = the bound of the child that schedules prmu[k] next.  Shared by the evaluate kernel below and the count
+// kernel of the fused expand (pfsp_wide_expand.cuh).  fc = this thread's column of PfspWideSmem::fc (stride
+// PW_THREADS).  Returns the parent's limit1, clamped to [-1, jobs-1].
+template <int KIND, int M, class Emit>
+__device__ __forceinline__ int pw_parent_bounds(const PfspWideTables& tab, const int32_t* node, int32_t* fc, int best,
+                                                Emit&& emit) {
+  const int jobs = tab.jobs;
+  const int limit1 = min(max(node[1], -1), jobs - 1);
+  const int32_t* prmu = node + 2;
+  int F[M], R[M];
+#pragma unroll
+  for (int j = 0; j < M; j++) {
+    F[j] = 0;
+    R[j] = tab.total[j];
+  }
+  if (KIND == 0 && limit1 < 0) {  // lb1_d on the root: front = min_heads (schedule_front, Bound_simple.chpl:53-57)
+#pragma unroll
+    for (int j = 0; j < M; j++) F[j] = tab.min_heads[j];
+  }
+  unsigned long long sched = 0;  // set_flags (Bound_johnson.chpl:179-186) as a bit mask
+  for (int i = 0; i <= limit1; i++) {  // schedule_front / add_forward (:29-62); remain = total - scheduled
+    const int job = prmu[i];
+    const int32_t* row = &tab.pj[job * PW_PSTRIDE];
+    sched |= 1ull << job;
+    F[0] += row[0];
+    R[0] -= row[0];
+#pragma unroll
+    for (int j = 1; j < M; j++) {
+      F[j] = max(F[j - 1], F[j]) + row[j];
+      R[j] -= row[j];
+    }
+  }
+  for (int k = limit1 + 1; k < jobs; k++) {
+    const int job = prmu[k];  // the child schedules prmu[k] next (prmu[depth] <=> prmu[k])
+    const int32_t* row = &tab.pj[job * PW_PSTRIDE];
+    int lb;
+    if constexpr (KIND == 0) {  // add_front_and_bound (:197-222)
+      lb = F[0] + R[0] + tab.min_tails[0];
+      int tmp0 = F[0] + row[0];
+#pragma unroll
+      for (int i = 1; i < M; i++) {
+        const int tmp1 = max(tmp0, F[i]);
+        lb = max(lb, tmp1 + R[i] + tab.min_tails[i]);
+        tmp0 = tmp1 + row[i];
+      }
+    } else if constexpr (KIND == 1) {  // lb1_bound on the child (:123-136): front_c, remain_c, running max
+      int fcj = F[0] + row[0];
+      int tmp0 = fcj + (R[0] - row[0]);
+      lb = tmp0 + tab.min_tails[0];
+#pragma unroll
+      for (int i = 1; i < M; i++) {
+        fcj = max(fcj, F[i]) + row[i];
+        const int tmp1 = max(tmp0, fcj + (R[i] - row[i]));
+        lb = max(lb, tmp1 + tab.min_tails[i]);
+        tmp0 = tmp1;
+      }
+    } else {  // lb2_bound (Bound_johnson.chpl:274-289): child front, flags, lb_makespan with early exit
+      int fcj = F[0] + row[0];
+      fc[0 * PW_THREADS] = fcj;
+#pragma unroll
+      for (int i = 1; i < M; i++) {
+        fcj = max(fcj, F[i]) + row[i];
+        fc[i * PW_THREADS] = fcj;
+      }
+      const unsigned long long flags = sched | (1ull << job);
+      lb = 0;
+      for (int l = 0; l < tab.pairs; l++) {
+        const uint32_t pw = tab.pair[l];
+        const int a = pw & 31u, b = (pw >> 5) & 31u;
+        int t0 = fc[a * PW_THREADS], t1 = fc[b * PW_THREADS];
+        const uint32_t* jp = &tab.jp[l * jobs];
+        for (int pos = 0; pos < jobs; pos++) {  // compute_cmax_johnson (:188-212)
+          const uint32_t e = jp[pos];
+          if (!((flags >> (e & 63u)) & 1ull)) {
+            t0 += (e >> 6) & 127u;
+            t1 = max(t1, t0 + static_cast<int>(e >> 20)) + static_cast<int>((e >> 13) & 127u);
+          }
+        }
+        const int c = max(t1 + static_cast<int>(pw >> 21), t0 + static_cast<int>((pw >> 10) & 2047u));
+        lb = max(lb, c);
+        if (lb > best) break;  // :232-236
+      }
+    }
+    emit(k, lb);
+  }
+  return limit1;
+}
+
+// the whole instance table into shared memory (lb1 / lb1_d never read the Johnson words); callers synchronise
+template <int KIND>
+__device__ __forceinline__ void pw_stage_tables(PfspWideTables* dst_tab, const PfspWideTables* __restrict__ tables) {
+  const uint4* src = reinterpret_cast<const uint4*>(tables);
+  uint4* dst = reinterpret_cast<uint4*>(dst_tab);
+  const int n16 = static_cast<int>((KIND == 2 ? sizeof(PfspWideTables) : offsetof(PfspWideTables, jp)) / 16);
+  for (int i = threadIdx.x; i < n16; i += blockDim.x) dst[i] = src[i];
+}
+
 template <int KIND, int M>
 __global__ void __launch_bounds__(PW_THREADS) pfsp_wide_kernel(const uint8_t* __restrict__ parents,
                                                               int32_t* __restrict__ bounds, long long count,
@@ -54,13 +153,7 @@ __global__ void __launch_bounds__(PW_THREADS) pfsp_wide_kernel(const uint8_t* __
   extern __shared__ __align__(128) uint8_t smem_raw[];
   PfspWideSmem& sm = *reinterpret_cast<PfspWideSmem*>(smem_raw);
   const int t = threadIdx.x;
-  {
-    const uint4* src = reinterpret_cast<const uint4*>(tables);
-    uint4* dst = reinterpret_cast<uint4*>(&sm.tab);
-    // (lb1 / lb1_d never read the Johnson words)
-    const int n16 = static_cast<int>((KIND == 2 ? sizeof(PfspWideTables) : offsetof(PfspWideTables, jp)) / 16);
-    for (int i = t; i < n16; i += PW_THREADS) dst[i] = src[i];
-  }
+  pw_stage_tables<KIND>(&sm.tab, tables);
   __syncthreads();
   const PfspWideTables& tab = sm.tab;
   const int jobs = tab.jobs;
@@ -75,86 +168,8 @@ __global__ void __launch_bounds__(PW_THREADS) pfsp_wide_kernel(const uint8_t* __
     }
     __syncthreads();
     if (t < np) {
-      const int32_t* node = sm.in + t * (PW_REC / 4);
-      const int limit1 = min(max(node[1], -1), jobs - 1);
-      const int32_t* prmu = node + 2;
-      int F[M], R[M];
-#pragma unroll
-      for (int j = 0; j < M; j++) {
-        F[j] = 0;
-        R[j] = tab.total[j];
-      }
-      if (KIND == 0 && limit1 < 0) {  // lb1_d on the root: front = min_heads (schedule_front, Bound_simple.chpl:53-57)
-#pragma unroll
-        for (int j = 0; j < M; j++) F[j] = tab.min_heads[j];
-      }
-      unsigned long long sched = 0;  // set_flags (Bound_johnson.chpl:179-186) as a bit mask
-      for (int i = 0; i <= limit1; i++) {  // schedule_front / add_forward (:29-62); remain = total - scheduled
-        const int job = prmu[i];
-        const int32_t* row = &tab.pj[job * PW_PSTRIDE];
-        sched |= 1ull << job;
-        F[0] += row[0];
-        R[0] -= row[0];
-#pragma unroll
-        for (int j = 1; j < M; j++) {
-          F[j] = max(F[j - 1], F[j]) + row[j];
-          R[j] -= row[j];
-        }
-      }
       int32_t* out = sm.out + t * jobs;
-      for (int k = limit1 + 1; k < jobs; k++) {
-        const int job = prmu[k];  // the child schedules prmu[k] next (prmu[depth] <=> prmu[k])
-        const int32_t* row = &tab.pj[job * PW_PSTRIDE];
-        int lb;
-        if constexpr (KIND == 0) {  // add_front_and_bound (:197-222)
-          lb = F[0] + R[0] + tab.min_tails[0];
-          int tmp0 = F[0] + row[0];
-#pragma unroll
-          for (int i = 1; i < M; i++) {
-            const int tmp1 = max(tmp0, F[i]);
-            lb = max(lb, tmp1 + R[i] + tab.min_tails[i]);
-            tmp0 = tmp1 + row[i];
-          }
-        } else if constexpr (KIND == 1) {  // lb1_bound on the child (:123-136): front_c, remain_c, running max
-          int fcj = F[0] + row[0];
-          int tmp0 = fcj + (R[0] - row[0]);
-          lb = tmp0 + tab.min_tails[0];
-#pragma unroll
-          for (int i = 1; i < M; i++) {
-            fcj = max(fcj, F[i]) + row[i];
-            const int tmp1 = max(tmp0, fcj + (R[i] - row[i]));
-            lb = max(lb, tmp1 + tab.min_tails[i]);
-            tmp0 = tmp1;
-          }
-        } else {  // lb2_bound (Bound_johnson.chpl:274-289): child front, flags, lb_makespan with early exit
-          int fcj = F[0] + row[0];
-          sm.fc[0 * PW_THREADS + t] = fcj;
-#pragma unroll
-          for (int i = 1; i < M; i++) {
-            fcj = max(fcj, F[i]) + row[i];
-            sm.fc[i * PW_THREADS + t] = fcj;
-          }
-          const unsigned long long flags = sched | (1ull << job);
-          lb = 0;
-          for (int l = 0; l < tab.pairs; l++) {
-            const uint32_t pw = tab.pair[l];
-            const int a = pw & 31u, b = (pw >> 5) & 31u;
-            int t0 = sm.fc[a * PW_THREADS + t], t1 = sm.fc[b * PW_THREADS + t];
-            const uint32_t* jp = &tab.jp[l * jobs];
-            for (int pos = 0; pos < jobs; pos++) {  // compute_cmax_johnson (:188-212)
-              const uint32_t e = jp[pos];
-              if (!((flags >> (e & 63u)) & 1ull)) {
-                t0 += (e >> 6) & 127u;
-                t1 = max(t1, t0 + static_cast<int>(e >> 20)) + static_cast<int>((e >> 13) & 127u);
-              }
-            }
-            const int c = max(t1 + static_cast<int>(pw >> 21), t0 + static_cast<int>((pw >> 10) & 2047u));
-            lb = max(lb, c);
-            if (lb > best) break;  // :232-236
-          }
-        }
-        out[k] = lb;
-      }
+      pw_parent_bounds<KIND, M>(tab, sm.in + t * (PW_REC / 4), sm.fc + t, best, [&](int k, int lb) { out[k] = lb; });
     }
     __syncthreads();
     // bounds of the tile: only the defined slots (k > limit1) are stored

@@ -24,6 +24,7 @@
 #include "nq_kernel.cuh"
 #include "pfsp_kernels.cuh"
 #include "pfsp_wide.cuh"
+#include "pfsp_wide_expand.cuh"
 #include "tsb200.h"
 
 namespace {
@@ -829,11 +830,16 @@ struct tsb_pfsp : Base {
   ExpandCtx ex;
   bool ex_attr[4] = {false, false, false, false};  // count lb1_d, lb1, lb2; build
   int ex_occ[4] = {0, 0, 0, 0};
+  bool wex_attr[4] = {false, false, false, false};  // the same for the 208-byte kernels (pfsp_wide_expand.cuh)
+  int wex_occ[4] = {0, 0, 0, 0};
   uint8_t* d_children = nullptr;
   size_t d_children_bytes = 0;
   DevicePool pool;
   uint64_t slow_rounds = 0;
   std::vector<tsb_pfsp_node> h_chunk, h_kids;  // slow path scratch
+  std::vector<tsb_pfsp_node50> h_chunk50, h_kids50;
+  size_t rec() const { return wide ? sizeof(tsb_pfsp_node50) : sizeof(tsb_pfsp_node); }  // bytes per node
+  int tile() const { return wide ? tsb::PW_TILE : tsb::PF_TILE; }                        // parents per expand tile
   std::vector<int32_t> h_bounds;
 };
 
@@ -997,11 +1003,49 @@ int pfsp_expand_m(tsb_pfsp* h, int lb_kind, const uint8_t* arena, const tsb::Exp
   return TSB_OK;
 }
 
+// 208-byte nodes (pfsp_wide_expand.cuh): count + build, one template per (bound, machines)
+template <int KIND, int M>
+int pfsp_wide_expand_km(tsb_pfsp* h, const uint8_t* arena, const tsb::ExpandParams& prm, uint8_t* children_d,
+                        cudaStream_t s) {
+  ExpandCtx& ex = h->ex;
+  const long long recs = static_cast<long long>(prm.n_tiles) * tsb::PW_TILE;
+  auto k1 = tsb::pfsp_wide_expand_count_kernel<KIND, M>;
+  auto k3 = tsb::pfsp_wide_expand_build_kernel;
+  const size_t smem1 = sizeof(tsb::PwCountSmem) + 128, smem3 = sizeof(tsb::PwBuildSmem) + 128;
+  if (!h->wex_attr[KIND]) {
+    TSB_CUDA(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem1)));
+    h->wex_attr[KIND] = true;
+  }
+  if (!h->wex_attr[3]) {
+    TSB_CUDA(cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem3)));
+    h->wex_attr[3] = true;
+  }
+  int g1 = 1, g3 = 1;
+  int rc = grid_for(k1, tsb::PW_THREADS, smem1, recs, tsb::PW_TILE, h->di.sms, &g1, &h->wex_occ[KIND]);
+  if (rc == TSB_OK) rc = grid_for(k3, tsb::PW_THREADS, smem3, recs, tsb::PW_TILE, h->di.sms, &g3, &h->wex_occ[3]);
+  if (rc != TSB_OK) return rc;
+  if ((prm.n_tiles + g3 - 1) / g3 > tsb::EXP_MAX_OWN) return TSB_EINVAL;
+  auto* cmask = reinterpret_cast<unsigned long long*>(ex.d_cmask);
+  k1<<<g1, tsb::PW_THREADS, smem1, s>>>(arena, prm, h->d_wtab, cmask, ex.d_tile, ex.d_st);
+  k3<<<g3, tsb::PW_THREADS, smem3, s>>>(arena, prm, cmask, ex.d_tile, children_d, ex.d_st, ex.d_res);
+  TSB_CUDA(cudaGetLastError());
+  h->launches += 2;
+  return TSB_OK;
+}
+template <int M>
+int pfsp_wide_expand_m(tsb_pfsp* h, int lb_kind, const uint8_t* arena, const tsb::ExpandParams& prm,
+                       uint8_t* children_d, cudaStream_t s) {
+  if (lb_kind == TSB_LB1_D) return pfsp_wide_expand_km<0, M>(h, arena, prm, children_d, s);
+  if (lb_kind == TSB_LB1) return pfsp_wide_expand_km<1, M>(h, arena, prm, children_d, s);
+  return pfsp_wide_expand_km<2, M>(h, arena, prm, children_d, s);
+}
+
 // generate_children of pfsp_gpu_chpl.chpl:273-303 on host arrays (the sequential rule, used by the slow path)
-void pfsp_generate_children_host(int jobs, const tsb_pfsp_node* parents, int size, const int32_t* bounds,
-                                 int64_t* best, std::vector<tsb_pfsp_node>* kids, uint64_t* sol) {
+template <class Node>
+void pfsp_generate_children_host(int jobs, const Node* parents, int size, const int32_t* bounds, int64_t* best,
+                                 std::vector<Node>* kids, uint64_t* sol) {
   for (int i = 0; i < size; i++) {
-    const tsb_pfsp_node& parent = parents[i];
+    const Node& parent = parents[i];
     const int depth = parent.depth;
     for (int j = parent.limit1 + 1; j < jobs; j++) {
       const int32_t lb = bounds[j + static_cast<size_t>(i) * jobs];
@@ -1009,7 +1053,7 @@ void pfsp_generate_children_host(int jobs, const tsb_pfsp_node* parents, int siz
         ++*sol;
         if (lb < *best) *best = lb;
       } else if (lb < *best) {
-        tsb_pfsp_node c = parent;
+        Node c = parent;
         c.depth = depth + 1;
         c.limit1 = parent.limit1 + 1;
         std::swap(c.prmu[depth], c.prmu[j]);
@@ -1019,21 +1063,48 @@ void pfsp_generate_children_host(int jobs, const tsb_pfsp_node* parents, int siz
   }
 }
 
+// the host half of the slow path: the chunk (d_in) and its bounds (d_out) back, the sequential rule, the children
+// to `children_d`
+template <class Node>
+int pfsp_slow_children(tsb_pfsp* h, std::vector<Node>& chunk, std::vector<Node>& kids, long long n,
+                       uint8_t* children_d, cudaStream_t s, int64_t* best, unsigned long long* n_children,
+                       unsigned long long* n_solutions) {
+  chunk.resize(static_cast<size_t>(n));
+  int rc = h->copy_d2h(chunk.data(), h->d_in, static_cast<size_t>(n) * sizeof(Node), s);
+  if (rc == TSB_OK) rc = h->copy_d2h(h->h_bounds.data(), h->d_out, static_cast<size_t>(n) * h->jobs * 4, s);
+  if (rc != TSB_OK) return rc;
+  kids.clear();
+  uint64_t sol = 0;
+  pfsp_generate_children_host(h->jobs, chunk.data(), static_cast<int>(n), h->h_bounds.data(), best, &kids, &sol);
+  rc = h->copy_h2d(children_d, kids.data(), kids.size() * sizeof(Node), s);
+  if (rc != TSB_OK) return rc;
+  *n_children = kids.size();
+  *n_solutions = sol;
+  return TSB_OK;
+}
+
 // One evaluate + generate_children round over `pieces` of `arena`; children packed at `children_d` (room for
 // n * jobs nodes).  *best is read and updated with the reference's semantics.  Synchronous.
 int pfsp_expand_round(tsb_pfsp* h, int lb_kind, const uint8_t* arena, const std::vector<PoolExtent>& pieces,
                       uint8_t* children_d, cudaStream_t s, int64_t* best, unsigned long long* n_children,
                       unsigned long long* n_solutions, bool early = false) {
   tsb::ExpandParams prm;
-  int rc = make_params(pieces, tsb::PF_TILE, &prm);
+  const int tile = h->tile();
+  int rc = make_params(pieces, tile, &prm);
   if (rc != TSB_OK) return rc;
   const int best_launch = clamp_best(*best);
   ExpandCtx& ex = h->ex;
-  rc = ex.reserve(std::max<long long>(prm.n_tiles, h->M_max / tsb::PF_TILE + 2 * tsb::EXP_MAX_PIECES), tsb::PF_TILE * 4, s);
+  // side array: one child mask per parent, 32-bit for 20 jobs, 64-bit for 50
+  rc = ex.reserve(std::max<long long>(prm.n_tiles, h->M_max / tile + 2 * tsb::EXP_MAX_PIECES),
+                  static_cast<long long>(tile) * (h->wide ? 8 : 4), s);
   if (rc != TSB_OK) return rc;
   prm.epoch = ++ex.epoch;
   prm.best = best_launch;
-  if (h->mt == 5)
+  if (h->wide)
+    rc = h->mt == 5 ? pfsp_wide_expand_m<5>(h, lb_kind, arena, prm, children_d, s)
+         : h->mt == 10 ? pfsp_wide_expand_m<10>(h, lb_kind, arena, prm, children_d, s)
+                       : pfsp_wide_expand_m<20>(h, lb_kind, arena, prm, children_d, s);
+  else if (h->mt == 5)
     rc = pfsp_expand_m<5>(h, lb_kind, arena, prm, children_d, s);
   else if (h->mt == 10)
     rc = pfsp_expand_m<10>(h, lb_kind, arena, prm, children_d, s);
@@ -1056,29 +1127,19 @@ int pfsp_expand_round(tsb_pfsp* h, int lb_kind, const uint8_t* arena, const std:
   long long n = 0;
   for (const PoolExtent& x : pieces) n += x.e - x.b;
   if (n > h->M_max) return TSB_EINVAL;  // (cannot happen: every entry point checks count <= M_max first)
+  const size_t rec = h->rec();
   long long at = 0;
   if (!(arena == h->d_in && pieces.size() == 1 && pieces[0].b == 0))
     for (const PoolExtent& x : pieces) {  // the chunk, contiguous
-      TSB_CUDA(cudaMemcpyAsync(h->d_in + at * sizeof(tsb_pfsp_node), arena + x.b * sizeof(tsb_pfsp_node),
-                               static_cast<size_t>(x.e - x.b) * sizeof(tsb_pfsp_node), cudaMemcpyDeviceToDevice, s));
+      TSB_CUDA(cudaMemcpyAsync(h->d_in + at * rec, arena + x.b * rec, static_cast<size_t>(x.e - x.b) * rec,
+                               cudaMemcpyDeviceToDevice, s));
       at += x.e - x.b;
     }
   rc = launch_pfsp(h, lb_kind, h->d_in, h->d_out, n, *best, s);
   if (rc != TSB_OK) return rc;
-  h->h_chunk.resize(static_cast<size_t>(n));
   h->h_bounds.resize(static_cast<size_t>(n) * h->jobs);
-  rc = h->copy_d2h(h->h_chunk.data(), h->d_in, static_cast<size_t>(n) * sizeof(tsb_pfsp_node), s);
-  if (rc == TSB_OK) rc = h->copy_d2h(h->h_bounds.data(), h->d_out, static_cast<size_t>(n) * h->jobs * 4, s);
-  if (rc != TSB_OK) return rc;
-  h->h_kids.clear();
-  uint64_t sol = 0;
-  pfsp_generate_children_host(h->jobs, h->h_chunk.data(), static_cast<int>(n), h->h_bounds.data(), best, &h->h_kids,
-                              &sol);
-  rc = h->copy_h2d(children_d, h->h_kids.data(), h->h_kids.size() * sizeof(tsb_pfsp_node), s);
-  if (rc != TSB_OK) return rc;
-  *n_children = h->h_kids.size();
-  *n_solutions = sol;
-  return TSB_OK;
+  return h->wide ? pfsp_slow_children(h, h->h_chunk50, h->h_kids50, n, children_d, s, best, n_children, n_solutions)
+                 : pfsp_slow_children(h, h->h_chunk, h->h_kids, n, children_d, s, best, n_children, n_solutions);
 }
 
 long long pfsp_pool_min_cap(const tsb_pfsp* h) {
@@ -1086,11 +1147,15 @@ long long pfsp_pool_min_cap(const tsb_pfsp* h) {
   return std::max<long long>(1LL << 20, 4LL * h->M_max * h->jobs);
 }
 void pfsp_pool_setup(tsb_pfsp* h) {
-  h->pool.rec = sizeof(tsb_pfsp_node);
-  h->pool.slack = static_cast<size_t>(tsb::PF_TILE) * sizeof(tsb_pfsp_node);
+  h->pool.rec = h->rec();
+  h->pool.slack = static_cast<size_t>(h->tile()) * h->rec();
 }
 
 }  // namespace
+
+__attribute__((visibility("hidden"))) int tsb_pfsp_handle_max_jobs(const tsb_pfsp* h) {
+  return h && h->wide ? TSB_MAX_JOBS_WIDE : TSB_MAX_JOBS;
+}
 
 // ============================================================================ exported C ABI
 extern "C" {
@@ -2038,8 +2103,8 @@ int tsb_pfsp_create(tsb_pfsp** out, int device, int jobs, int machines, int M_ma
 }
 
 // The reference built with MAX_JOBS = max_jobs (lib/pfsp/PFSP_node.chpl:7): 20 = tsb_pfsp_create; 50 = 208-byte nodes,
-// jobs == 50 instances (ta031..ta060), evaluated by the general kernels of pfsp_wide.cuh (evaluate / evaluate_device
-// only: the fused expand and the device pool are specialised for 20 jobs)
+// jobs == 50 instances (ta031..ta060), evaluated by the general kernels of pfsp_wide.cuh; the fused expand and the
+// device pool run the 208-byte kernels of pfsp_wide_expand.cuh
 int tsb_pfsp_create_wide(tsb_pfsp** out, int device, int max_jobs, int jobs, int machines, int M_max, const int32_t* p_times,
                          const int32_t* min_heads, const int32_t* min_tails, int nb_pairs, const int32_t* johnson,
                          const int32_t* lags, const int32_t* mp0, const int32_t* mp1, const int32_t* mp_order) {
@@ -2182,13 +2247,14 @@ uint64_t tsb_pfsp_slow_rounds(const tsb_pfsp* h) { return h ? h->slow_rounds : 0
 
 int tsb_pfsp_expand_device(tsb_pfsp* h, int lb_kind, const void* parents_d, int count, int64_t* best,
                            void* children_d, uint64_t* n_children, uint64_t* n_solutions, void* stream) {
-  if (h && h->wide) return TSB_EUNSUPPORTED;  // (the fused expand / device pool exist for MAX_JOBS = 20 only)
   if (!h || count < 0 || lb_kind < 0 || lb_kind > 2 || !best || !n_children || !n_solutions) return TSB_EINVAL;
   if (lb_kind == TSB_LB2 && h->pairs == 0) return TSB_EINVAL;
   *n_children = *n_solutions = 0;
   if (count == 0) return TSB_OK;
   if (!parents_d || !children_d || count > h->M_max) return TSB_EINVAL;
-  if ((reinterpret_cast<uintptr_t>(parents_d) & 15) || (reinterpret_cast<uintptr_t>(children_d) & 7)) return TSB_EALIGN;
+  // (208-byte children are written by whole-image TMA stores: 16-byte aligned like the parents)
+  if ((reinterpret_cast<uintptr_t>(parents_d) & 15) || (reinterpret_cast<uintptr_t>(children_d) & (h->wide ? 15 : 7)))
+    return TSB_EALIGN;
   TSB_CUDA(cudaSetDevice(h->device));
   unsigned long long nc = 0, ns = 0;
   const std::vector<PoolExtent> pieces{{0, count}};
@@ -2202,7 +2268,6 @@ int tsb_pfsp_expand_device(tsb_pfsp* h, int lb_kind, const void* parents_d, int 
 
 int tsb_pfsp_expand(tsb_pfsp* h, int lb_kind, const void* parents, int count, int64_t* best, void* children,
                     uint64_t capacity, uint64_t* n_children, uint64_t* n_solutions) {
-  if (h && h->wide) return TSB_EUNSUPPORTED;  // (the fused expand / device pool exist for MAX_JOBS = 20 only)
   if (!h || count < 0 || count > h->M_max || lb_kind < 0 || lb_kind > 2 || !best || !n_children || !n_solutions)
     return TSB_EINVAL;
   if (lb_kind == TSB_LB2 && h->pairs == 0) return TSB_EINVAL;
@@ -2210,7 +2275,8 @@ int tsb_pfsp_expand(tsb_pfsp* h, int lb_kind, const void* parents, int count, in
   if (count == 0) return TSB_OK;
   if (!parents || !children) return TSB_EINVAL;
   TSB_CUDA(cudaSetDevice(h->device));
-  const size_t need = static_cast<size_t>(h->M_max) * h->jobs * sizeof(tsb_pfsp_node) + 64;
+  const size_t rec = h->rec();
+  const size_t need = static_cast<size_t>(h->M_max) * h->jobs * rec + 64;
   if (h->d_children_bytes < need) {
     if (h->d_children) cudaFree(h->d_children);
     h->d_children = nullptr;
@@ -2218,7 +2284,7 @@ int tsb_pfsp_expand(tsb_pfsp* h, int lb_kind, const void* parents, int count, in
     TSB_CUDA(cudaMalloc(&h->d_children, need));
     h->d_children_bytes = need;
   }
-  int rc = h->copy_h2d(h->d_in, parents, sizeof(tsb_pfsp_node) * static_cast<size_t>(count), h->stream);
+  int rc = h->copy_h2d(h->d_in, parents, rec * static_cast<size_t>(count), h->stream);
   if (rc != TSB_OK) return rc;
   unsigned long long nc = 0, ns = 0;
   const std::vector<PoolExtent> pieces{{0, count}};
@@ -2227,11 +2293,10 @@ int tsb_pfsp_expand(tsb_pfsp* h, int lb_kind, const void* parents, int count, in
   *n_children = nc;
   *n_solutions = ns;
   if (nc > capacity) return TSB_ENOMEM;
-  return h->copy_d2h(children, h->d_children, nc * sizeof(tsb_pfsp_node), h->stream);
+  return h->copy_d2h(children, h->d_children, nc * rec, h->stream);
 }
 
 int tsb_pfsp_pool_push(tsb_pfsp* h, const void* nodes, int64_t n) {
-  if (h && h->wide) return TSB_EUNSUPPORTED;  // (the fused expand / device pool exist for MAX_JOBS = 20 only)
   if (!h || n < 0 || (n && !nodes)) return TSB_EINVAL;
   TSB_CUDA(cudaSetDevice(h->device));
   pfsp_pool_setup(h);
@@ -2239,8 +2304,7 @@ int tsb_pfsp_pool_push(tsb_pfsp* h, const void* nodes, int64_t n) {
   if (rc != TSB_OK) return rc;
   if (n == 0) return TSB_OK;
   const long long at = h->pool.top();
-  rc = h->copy_h2d(h->pool.arena[h->pool.cur] + at * sizeof(tsb_pfsp_node), nodes,
-                   static_cast<size_t>(n) * sizeof(tsb_pfsp_node), h->stream);
+  rc = h->copy_h2d(h->pool.arena[h->pool.cur] + at * h->rec(), nodes, static_cast<size_t>(n) * h->rec(), h->stream);
   if (rc != TSB_OK) return rc;
   if (h->pool.ext.empty())
     h->pool.ext.push_back({at, at + n});
@@ -2254,7 +2318,6 @@ int64_t tsb_pfsp_pool_size(const tsb_pfsp* h) { return h ? h->pool.size : -1; }
 
 int tsb_pfsp_pool_step(tsb_pfsp* h, int lb_kind, int m, int M, int64_t* best, int64_t* n_parents,
                        uint64_t* n_children, uint64_t* n_solutions) {
-  if (h && h->wide) return TSB_EUNSUPPORTED;  // (the fused expand / device pool exist for MAX_JOBS = 20 only)
   if (!h || lb_kind < 0 || lb_kind > 2 || m < 1 || M < 1 || M > h->M_max || !best || !n_parents || !n_children ||
       !n_solutions)
     return TSB_EINVAL;
@@ -2272,10 +2335,11 @@ int tsb_pfsp_pool_step(tsb_pfsp* h, int lb_kind, int m, int M, int64_t* best, in
   if (rc == TSB_OK) rc = p.reserve(h->stream, n * h->jobs + 2, pfsp_pool_min_cap(h));
   if (rc != TSB_OK) return rc;
   pool_top_pieces(p, n, &pieces);
-  const long long top = (p.top() + 1) & ~1LL;  // children start on a 16-byte boundary (88 B records)
+  // children start on a 16-byte boundary (88-byte records: an even position; 208 = 13 * 16: any position)
+  const long long top = h->wide ? p.top() : (p.top() + 1) & ~1LL;
   unsigned long long nc = 0, ns = 0;
   uint8_t* arena = p.arena[p.cur];
-  rc = pfsp_expand_round(h, lb_kind, arena, pieces, arena + top * sizeof(tsb_pfsp_node), h->stream, best, &nc, &ns,
+  rc = pfsp_expand_round(h, lb_kind, arena, pieces, arena + top * h->rec(), h->stream, best, &nc, &ns,
                          /*early=*/true);
   if (rc != TSB_OK) return rc;
   pool_pop(p, n);
@@ -2308,9 +2372,8 @@ int tsb_pfsp_pool_drain(tsb_pfsp* h, void* nodes, int64_t capacity, int64_t* n) 
   TSB_CUDA(cudaSetDevice(h->device));
   long long at = 0;
   for (const PoolExtent& x : p.ext) {
-    int rc = h->copy_d2h(static_cast<uint8_t*>(nodes) + at * sizeof(tsb_pfsp_node),
-                         p.arena[p.cur] + x.b * sizeof(tsb_pfsp_node),
-                         static_cast<size_t>(x.e - x.b) * sizeof(tsb_pfsp_node), h->stream);
+    int rc = h->copy_d2h(static_cast<uint8_t*>(nodes) + at * h->rec(), p.arena[p.cur] + x.b * h->rec(),
+                         static_cast<size_t>(x.e - x.b) * h->rec(), h->stream);
     if (rc != TSB_OK) return rc;
     at += x.e - x.b;
   }

@@ -23,6 +23,9 @@
 
 #include "tsb200.h"
 
+// MAX_JOBS of the build a handle emulates: 20 or 50 (tsb200_api.cu; internal to the library)
+__attribute__((visibility("hidden"))) int tsb_pfsp_handle_max_jobs(const tsb_pfsp* h);
+
 namespace {
 
 // ---- Taillard benchmark data (seeds and best-known makespans of ta001..ta120, Taillard 1993;
@@ -526,9 +529,25 @@ int64_t unif(int64_t& seed, int64_t low, int64_t high) {  // lib/pfsp/Taillard.c
   return low + static_cast<int64_t>(v * static_cast<double>(high - low + 1));
 }
 
+// the two builds of the reference: MAX_JOBS = 20 (tsb_pfsp_tables, 88-byte nodes) and MAX_JOBS = 50
+// (tsb_pfsp_tables50, 208-byte nodes, ta031..ta060)
+template <class Node>
+constexpr int max_jobs_of() {
+  return static_cast<int>(sizeof(Node::prmu) / sizeof(int32_t));
+}
+inline int pfsp_tables_for(tsb_pfsp_tables* t, int inst) { return tsb_pfsp_tables_build(t, inst); }
+inline int pfsp_tables_for(tsb_pfsp_tables50* t, int inst) { return tsb_pfsp_tables50_build(t, inst, TSB_LB2_FULL); }
+inline int pfsp_create_for(tsb_pfsp** h, int device, int M, const tsb_pfsp_tables* t) {
+  return tsb_pfsp_create_from_tables(h, device, M, t);
+}
+inline int pfsp_create_for(tsb_pfsp** h, int device, int M, const tsb_pfsp_tables50* t) {
+  return tsb_pfsp_create50_from_tables(h, device, M, t);
+}
+
+template <class Tables>
 struct HostBounds {  // CPU bounds used by decompose in steps 1 and 3 (pfsp_gpu_chpl.chpl:88-189)
-  const tsb_pfsp_tables& t;
-  explicit HostBounds(const tsb_pfsp_tables& tt) : t(tt) {}
+  const Tables& t;
+  explicit HostBounds(const Tables& tt) : t(tt) {}
   void front_of(const int32_t* prmu, int limit1, int32_t* F) const {  // schedule_front
     const int N = t.jobs, M = t.machines;
     if (limit1 == -1) {
@@ -566,7 +585,7 @@ struct HostBounds {  // CPU bounds used by decompose in steps 1 and 3 (pfsp_gpu_
     int32_t F[TSB_MAX_MACHINES], R[TSB_MAX_MACHINES];
     front_of(prmu, limit1, F);
     remain_of(prmu, limit1, R);
-    std::fill(lb_begin, lb_begin + TSB_MAX_JOBS, 0);
+    std::fill(lb_begin, lb_begin + N, 0);
     for (int i = limit1 + 1; i < N; i++) {
       const int job = prmu[i];
       int32_t lb = F[0] + R[0] + t.min_tails[0], tmp0 = F[0] + t.p_times[job];
@@ -582,15 +601,15 @@ struct HostBounds {  // CPU bounds used by decompose in steps 1 and 3 (pfsp_gpu_
     const int N = t.jobs;
     int32_t F[TSB_MAX_MACHINES];
     front_of(prmu, limit1, F);
-    uint32_t sched = 0;
-    for (int j = 0; j <= limit1; j++) sched |= 1u << prmu[j];
+    uint64_t sched = 0;  // (64-bit: jobs up to 50)
+    for (int j = 0; j <= limit1; j++) sched |= 1ull << prmu[j];
     int32_t lb = 0;
     for (int l = 0; l < t.pairs; l++) {
       const int i = t.mp_order[l], a = t.mp0[i], b = t.mp1[i];
       int32_t t0 = F[a], t1 = F[b];
       for (int j = 0; j < N; j++) {
         const int job = t.johnson[i * N + j];
-        if (!((sched >> job) & 1u)) {
+        if (!((sched >> job) & 1ull)) {
           t0 += t.p_times[a * N + job];
           t1 = std::max(t1, t0 + t.lags[i * N + job]) + t.p_times[b * N + job];
         }
@@ -602,7 +621,8 @@ struct HostBounds {  // CPU bounds used by decompose in steps 1 and 3 (pfsp_gpu_
   }
 };
 
-inline void pfsp_child(const tsb_pfsp_node& parent, int i, tsb_pfsp_node& c) {
+template <class Node>
+inline void pfsp_child(const Node& parent, int i, Node& c) {
   c = parent;
   c.depth = parent.depth + 1;
   c.limit1 = parent.limit1 + 1;
@@ -610,13 +630,14 @@ inline void pfsp_child(const tsb_pfsp_node& parent, int i, tsb_pfsp_node& c) {
 }
 
 // decompose (pfsp_gpu_chpl.chpl:88-189)
-void pfsp_decompose(const HostBounds& hb, int lb_kind, const tsb_pfsp_node& parent, uint64_t& tree,
-                    uint64_t& sol, int64_t& best, Pool<tsb_pfsp_node>& pool) {
+template <class Tables, class Node>
+void pfsp_decompose(const HostBounds<Tables>& hb, int lb_kind, const Node& parent, uint64_t& tree, uint64_t& sol,
+                    int64_t& best, Pool<Node>& pool) {
   const int jobs = hb.t.jobs;
-  int32_t lb_begin[TSB_MAX_JOBS];
+  int32_t lb_begin[max_jobs_of<Node>()];
   if (lb_kind == TSB_LB1_D) hb.lb1_children(parent.prmu, parent.limit1, lb_begin);
   for (int i = parent.limit1 + 1; i < jobs; i++) {
-    tsb_pfsp_node c;
+    Node c;
     pfsp_child(parent, i, c);
     const int32_t lb = lb_kind == TSB_LB1_D ? lb_begin[parent.prmu[i]]
                        : lb_kind == TSB_LB1 ? hb.lb1(c.prmu, c.limit1)
@@ -632,10 +653,11 @@ void pfsp_decompose(const HostBounds& hb, int lb_kind, const tsb_pfsp_node& pare
 }
 
 // generate_children (pfsp_gpu_chpl.chpl:273-303)
-void pfsp_generate_children(int jobs, const tsb_pfsp_node* parents, int size, const int32_t* bounds,
-                            uint64_t& tree, uint64_t& sol, int64_t& best, Pool<tsb_pfsp_node>& pool) {
+template <class Node>
+void pfsp_generate_children(int jobs, const Node* parents, int size, const int32_t* bounds, uint64_t& tree,
+                            uint64_t& sol, int64_t& best, Pool<Node>& pool) {
   for (int i = 0; i < size; i++) {
-    const tsb_pfsp_node& parent = parents[i];
+    const Node& parent = parents[i];
     const int depth = parent.depth;
     for (int j = parent.limit1 + 1; j < jobs; j++) {
       const int32_t lb = bounds[j + static_cast<size_t>(i) * jobs];
@@ -643,7 +665,7 @@ void pfsp_generate_children(int jobs, const tsb_pfsp_node* parents, int size, co
         ++sol;
         if (lb < best) best = lb;
       } else if (lb < best) {
-        tsb_pfsp_node c;
+        Node c;
         pfsp_child(parent, j, c);
         pool.pushBack(c);
         ++tree;
@@ -652,16 +674,16 @@ void pfsp_generate_children(int jobs, const tsb_pfsp_node* parents, int size, co
   }
 }
 
-void pfsp_gpu_task(int device, const tsb_pfsp_tables& t, int lb_kind, int m, int M, Pool<tsb_pfsp_node>& pool,
-                   GpuTaskResult& r) {
+template <class Tables, class Node>
+void pfsp_gpu_task(int device, const Tables& t, int lb_kind, int m, int M, Pool<Node>& pool, GpuTaskResult& r) {
   tsb_pfsp* h = nullptr;
-  r.rc = tsb_pfsp_create_from_tables(&h, device, M, &t);
+  r.rc = pfsp_create_for(&h, device, M, &t);
   if (r.rc != TSB_OK) return;
   const int jobs = t.jobs;
-  std::vector<tsb_pfsp_node> parents(M);
+  std::vector<Node> parents(M);
   std::vector<int32_t> bounds(static_cast<size_t>(M) * jobs);
   // the chunk arrays live for the whole step 2 (pfsp_gpu_chpl.chpl:355-356): page-lock them once
-  tsb_pfsp_register_host(h, parents.data(), parents.size() * sizeof(tsb_pfsp_node));
+  tsb_pfsp_register_host(h, parents.data(), parents.size() * sizeof(Node));
   tsb_pfsp_register_host(h, bounds.data(), bounds.size() * sizeof(int32_t));
   for (;;) {
     const int n = pool.popBackBulk(m, M, parents.data());
@@ -677,7 +699,8 @@ void pfsp_gpu_task(int device, const tsb_pfsp_tables& t, int lb_kind, int m, int
 }
 
 // the same loop with the task's pool resident on the device (tsb_pfsp_pool_*)
-void pfsp_devpool_on(tsb_pfsp* h, int lb_kind, int m, int M, Pool<tsb_pfsp_node>& pool, GpuTaskResult& r,
+template <class Node>
+void pfsp_devpool_on(tsb_pfsp* h, int lb_kind, int m, int M, Pool<Node>& pool, GpuTaskResult& r,
                      StealBoard* sb = nullptr, int me = 0) {
   const uint64_t l0 = tsb_pfsp_kernel_launches(h);
   r.rc = tsb_pfsp_pool_push(h, &pool.el[pool.front], static_cast<int64_t>(pool.size));
@@ -709,17 +732,18 @@ void pfsp_devpool_on(tsb_pfsp* h, int lb_kind, int m, int M, Pool<tsb_pfsp_node>
   if (r.rc != TSB_OK) board_abort(sb, me);
   if (r.rc == TSB_OK) {
     const int64_t left = tsb_pfsp_pool_size(h);
-    std::vector<tsb_pfsp_node> rest(static_cast<size_t>(left) + 1);
+    std::vector<Node> rest(static_cast<size_t>(left) + 1);
     int64_t n = 0;
     r.rc = tsb_pfsp_pool_drain(h, rest.data(), left, &n);
     for (int64_t i = 0; i < n && r.rc == TSB_OK; i++) pool.pushBack(rest[i]);
   }
   r.launches = tsb_pfsp_kernel_launches(h) - l0;
 }
-void pfsp_devpool_task(int device, const tsb_pfsp_tables& t, int lb_kind, int m, int M, Pool<tsb_pfsp_node>& pool,
-                       GpuTaskResult& r, StealBoard* sb = nullptr, int me = 0) {
+template <class Tables, class Node>
+void pfsp_devpool_task(int device, const Tables& t, int lb_kind, int m, int M, Pool<Node>& pool, GpuTaskResult& r,
+                       StealBoard* sb = nullptr, int me = 0) {
   tsb_pfsp* h = nullptr;
-  r.rc = tsb_pfsp_create_from_tables(&h, device, M, &t);
+  r.rc = pfsp_create_for(&h, device, M, &t);
   if (r.rc != TSB_OK) {
     if (sb) sb->publish_handle(me, nullptr, 0);
     return;
@@ -727,8 +751,9 @@ void pfsp_devpool_task(int device, const tsb_pfsp_tables& t, int lb_kind, int m,
   pfsp_devpool_on(h, lb_kind, m, M, pool, r, sb, me);
   tsb_pfsp_destroy(h);
 }
-void pfsp_gpu_task_nosteal(int device, const tsb_pfsp_tables& t, int lb_kind, int m, int M, Pool<tsb_pfsp_node>& pool,
-                           GpuTaskResult& r, StealBoard*, int) {
+template <class Tables, class Node>
+void pfsp_gpu_task_nosteal(int device, const Tables& t, int lb_kind, int m, int M, Pool<Node>& pool, GpuTaskResult& r,
+                           StealBoard*, int) {
   pfsp_gpu_task(device, t, lb_kind, m, M, pool, r);
 }
 
@@ -975,26 +1000,31 @@ static int nq_search_device_impl(int N, int g, int m, int M, int D, int part, in
   return TSB_OK;
 }
 
+}  // extern "C"
+
+// Tables / Node: the build of the reference the search emulates (tsb_pfsp_tables + tsb_pfsp_node: MAX_JOBS = 20;
+// tsb_pfsp_tables50 + tsb_pfsp_node50: MAX_JOBS = 50)
+template <class Tables, class Node>
 static int pfsp_search_impl(int inst, int lb_kind, int ub, int m, int M, int D, bool devpool, int part, int device,
                             tsb_pfsp* on, tsb_search_stats* out) {
   if (!out || lb_kind < 0 || lb_kind > 2 || (ub != 0 && ub != 1) || m < 1 || M < 1 || D < 1 || D > 8 || part >= D)
     return TSB_EINVAL;
   std::memset(out, 0, sizeof(*out));
-  std::vector<tsb_pfsp_tables> tv(1);
-  tsb_pfsp_tables& t = tv[0];
-  int rc = tsb_pfsp_tables_build(&t, inst);
+  std::vector<Tables> tv(1);
+  Tables& t = tv[0];
+  int rc = pfsp_tables_for(&t, inst);
   if (rc != TSB_OK) return rc;
   if (!on)
     if (rc = tsb_init_devices(part < 0 ? D : device + 1); rc != TSB_OK) return rc;  // contexts exist before the timers start
-  HostBounds hb(t);
+  HostBounds<Tables> hb(t);
   int64_t best = ub == 1 ? tsb_taillard_best_ub(inst) : INT64_MAX;  // pfsp_gpu_chpl.chpl:37
-  Pool<tsb_pfsp_node> pool;
-  tsb_pfsp_node root{};
+  Pool<Node> pool;
+  Node root{};
   root.limit1 = -1;
   for (int i = 0; i < t.jobs; i++) root.prmu[i] = i;
   pool.pushBack(root);
   uint64_t tree = 0, sol = 0;
-  tsb_pfsp_node parent;
+  Node parent;
   double t0 = now_s();
   while (pool.size < static_cast<size_t>(D) * m) {
     if (!pool.popFront(parent)) break;
@@ -1005,12 +1035,12 @@ static int pfsp_search_impl(int inst, int lb_kind, int ub, int m, int M, int D, 
   std::vector<GpuTaskResult> res(D);
   const int ndev = std::max(1, tsb_device_count());
   for (auto& r : res) r.best = best;  // per-task best_l = best (pfsp_multigpu_chpl.chpl:384)
-  auto task = devpool ? pfsp_devpool_task : pfsp_gpu_task_nosteal;
+  auto task = devpool ? pfsp_devpool_task<Tables, Node> : pfsp_gpu_task_nosteal<Tables, Node>;
   if (on) {
     pfsp_devpool_on(on, lb_kind, m, M, pool, res[0]);
   } else if (part >= 0) {  // one task of the split (see nq_search_device_impl)
     if (part != 0) tree = sol = 0;
-    std::vector<Pool<tsb_pfsp_node>> multi;
+    std::vector<Pool<Node>> multi;
     if (D == 1) {
       multi.resize(1);
       std::swap(multi[0], pool);
@@ -1022,7 +1052,7 @@ static int pfsp_search_impl(int inst, int lb_kind, int ub, int m, int M, int D, 
   } else if (D == 1) {
     task(0, t, lb_kind, m, M, pool, res[0], nullptr, 0);
   } else {
-    std::vector<Pool<tsb_pfsp_node>> multi;
+    std::vector<Pool<Node>> multi;
     static_split(pool, D, multi);
     StealBoard board(D);
     // (stealing keeps the counts only when `best` is constant: --ub 1, SURVEY A.6)
@@ -1058,6 +1088,8 @@ static int pfsp_search_impl(int inst, int lb_kind, int ub, int m, int M, int D, 
   return TSB_OK;
 }
 
+extern "C" {
+
 // step 1 of the drivers alone (nqueens_gpu_chpl.chpl:169-175): breadth-first from the root until the pool holds
 // min_size nodes; the pool, in order, and what was explored on the way
 void tsb_release_cached_handles(void) { nq_handle_cache().clear(); }
@@ -1091,19 +1123,43 @@ int tsb_nq_search_on(tsb_nq* h, int N, int m, int M, tsb_search_stats* out) {
   return nq_search_device_impl(N, 1, m, M, 1, -1, 0, h, out);
 }
 int tsb_pfsp_search(int inst, int lb_kind, int ub, int m, int M, int D, tsb_search_stats* out) {
-  return pfsp_search_impl(inst, lb_kind, ub, m, M, D, false, -1, 0, nullptr, out);
+  return pfsp_search_impl<tsb_pfsp_tables, tsb_pfsp_node>(inst, lb_kind, ub, m, M, D, false, -1, 0, nullptr, out);
 }
 int tsb_pfsp_search_device(int inst, int lb_kind, int ub, int m, int M, int D, tsb_search_stats* out) {
-  return pfsp_search_impl(inst, lb_kind, ub, m, M, D, true, -1, 0, nullptr, out);
+  return pfsp_search_impl<tsb_pfsp_tables, tsb_pfsp_node>(inst, lb_kind, ub, m, M, D, true, -1, 0, nullptr, out);
 }
 int tsb_pfsp_search_device_part(int inst, int lb_kind, int ub, int m, int M, int D, int part, int device,
                                 tsb_search_stats* out) {
   if (part < 0) return TSB_EINVAL;
-  return pfsp_search_impl(inst, lb_kind, ub, m, M, D, true, part, device, nullptr, out);
+  return pfsp_search_impl<tsb_pfsp_tables, tsb_pfsp_node>(inst, lb_kind, ub, m, M, D, true, part, device, nullptr, out);
 }
 int tsb_pfsp_search_on(tsb_pfsp* h, int inst, int lb_kind, int ub, int m, int M, tsb_search_stats* out) {
   if (!h) return TSB_EINVAL;
-  return pfsp_search_impl(inst, lb_kind, ub, m, M, 1, true, -1, 0, h, out);
+  if (tsb_pfsp_handle_max_jobs(h) == TSB_MAX_JOBS_WIDE) {
+    if (inst < 1 || inst > 120) return TSB_EINVAL;
+    if (tsb_taillard_nb_jobs(inst) != TSB_MAX_JOBS_WIDE) return TSB_EUNSUPPORTED;  // the handle's build takes 50 jobs
+    return pfsp_search_impl<tsb_pfsp_tables50, tsb_pfsp_node50>(inst, lb_kind, ub, m, M, 1, true, -1, 0, h, out);
+  }
+  return pfsp_search_impl<tsb_pfsp_tables, tsb_pfsp_node>(inst, lb_kind, ub, m, M, 1, true, -1, 0, h, out);
+}
+
+// the search as a build of the reference with MAX_JOBS = max_jobs runs it: 20 = tsb_pfsp_search[_device]; 50 =
+// 208-byte nodes, ta031..ta060.  Everything is validated before any device is touched.
+static int pfsp_search_wide(int max_jobs, int inst, int lb_kind, int ub, int m, int M, int D, bool devpool,
+                            tsb_search_stats* out) {
+  if (max_jobs == TSB_MAX_JOBS)
+    return pfsp_search_impl<tsb_pfsp_tables, tsb_pfsp_node>(inst, lb_kind, ub, m, M, D, devpool, -1, 0, nullptr, out);
+  if (max_jobs != TSB_MAX_JOBS_WIDE) return TSB_EUNSUPPORTED;
+  if (inst < 1 || inst > 120) return TSB_EINVAL;
+  if (tsb_taillard_nb_jobs(inst) != TSB_MAX_JOBS_WIDE) return TSB_EUNSUPPORTED;  // (jobs == MAX_JOBS, as for handles)
+  return pfsp_search_impl<tsb_pfsp_tables50, tsb_pfsp_node50>(inst, lb_kind, ub, m, M, D, devpool, -1, 0, nullptr, out);
+}
+int tsb_pfsp_search_wide(int max_jobs, int inst, int lb_kind, int ub, int m, int M, int D, tsb_search_stats* out) {
+  return pfsp_search_wide(max_jobs, inst, lb_kind, ub, m, M, D, false, out);
+}
+int tsb_pfsp_search_device_wide(int max_jobs, int inst, int lb_kind, int ub, int m, int M, int D,
+                                tsb_search_stats* out) {
+  return pfsp_search_wide(max_jobs, inst, lb_kind, ub, m, M, D, true, out);
 }
 
 }  // extern "C"

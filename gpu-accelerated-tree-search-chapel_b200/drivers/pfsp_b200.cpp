@@ -1,6 +1,7 @@
 // pfsp_b200 — C++ stand-in for pfsp_gpu_chpl / pfsp_multigpu_chpl.  Same CLI (--inst --lb --ub --m --M
 // --D; README.md:47-87), same defaults (pfsp_multigpu_chpl.chpl:24-30: inst 14, lb "lb1", ub 1), same
-// result lines (pfsp_gpu_chpl.chpl:66-77).  --lb takes the Chapel spelling lb1 | lb1_d | lb2.
+// result lines (pfsp_gpu_chpl.chpl:66-77).  --lb takes the Chapel spelling lb1 | lb1_d | lb2.  --inst 31..60 (50 jobs)
+// runs as the reference built with `-sMAX_JOBS=50` (lib/pfsp/PFSP_node.chpl:7) does: 208-byte nodes.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -39,8 +40,15 @@ int main(int argc, char** argv) {
               "Lower bound function: %s\nBranching rule: fwd\n=================================================\n",
               D > 1 ? "Multi-GPU" : "Single-GPU", inst, tsb_taillard_nb_machines(inst), tsb_taillard_nb_jobs(inst),
               ub ? "opt" : "inf", lbs);
+  if (tsb_taillard_nb_jobs(inst) > TSB_MAX_JOBS_WIDE) {
+    std::fprintf(stderr, "Error: ta%03d has %d jobs; this build takes up to %d (ta001..ta060)\n", inst,
+                 tsb_taillard_nb_jobs(inst), TSB_MAX_JOBS_WIDE);
+    return 2;
+  }
+  const int max_jobs = tsb_taillard_nb_jobs(inst) > TSB_MAX_JOBS ? TSB_MAX_JOBS_WIDE : TSB_MAX_JOBS;
   tsb_search_stats st;
-  const int rc = devpool ? tsb_pfsp_search_device(inst, lb, ub, m, M, D, &st) : tsb_pfsp_search(inst, lb, ub, m, M, D, &st);
+  const int rc = devpool ? tsb_pfsp_search_device_wide(max_jobs, inst, lb, ub, m, M, D, &st)
+                         : tsb_pfsp_search_wide(max_jobs, inst, lb, ub, m, M, D, &st);
   if (rc != TSB_OK) {
     std::fprintf(stderr, "tsb_pfsp_search: %s (%s)\n", tsb_strerror(rc), tsb_last_cuda_error());
     return 3;

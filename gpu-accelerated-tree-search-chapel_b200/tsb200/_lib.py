@@ -122,6 +122,8 @@ SYMBOLS = {
     "tsb_nq_search_device": (_i, [_i, _i, _i, _i, _i, C.POINTER(SearchStats)]),
     "tsb_pfsp_search": (_i, [_i, _i, _i, _i, _i, _i, C.POINTER(SearchStats)]),
     "tsb_pfsp_search_device": (_i, [_i, _i, _i, _i, _i, _i, C.POINTER(SearchStats)]),
+    "tsb_pfsp_search_wide": (_i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(SearchStats)]),
+    "tsb_pfsp_search_device_wide": (_i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(SearchStats)]),
     "tsb_nq_search_on": (_i, [_vp, _i, _i, _i, C.POINTER(SearchStats)]),
     "tsb_pfsp_search_on": (_i, [_vp, _i, _i, _i, _i, _i, C.POINTER(SearchStats)]),
     "tsb_nq_search_device_part": (_i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(SearchStats)]),

@@ -5,7 +5,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import LB1, LB1_D, LB2, PfspTables, PfspTables50, SearchStats, check, lib
+from ._lib import EINVAL, LB1, LB1_D, LB2, PfspTables, PfspTables50, SearchStats, TsbError, check, lib
 
 # lib/pfsp/PFSP_node.chpl:9-12
 PFSP_NODE_DTYPE = np.dtype([("depth", np.int32), ("limit1", np.int32), ("prmu", np.int32, (20,))])
@@ -36,9 +36,14 @@ def taillard_tables50(inst: int, variant="full") -> PfspTables50:
     return t
 
 
+def _max_jobs(inst: int) -> int:
+    """MAX_JOBS of the reference build that runs `inst`: 20 for ta001..ta030, 50 for ta031..ta060"""
+    return 50 if lib().tsb_taillard_nb_jobs(inst) == 50 else 20
+
+
 class PfspEvaluator:
     """Owns parents_d / bounds_d / lbound1_d / lbound2_d of pfsp_gpu_chpl.chpl:359-371.  Instances with more than
-    20 jobs (ta031..ta060) create a MAX_JOBS = 50 handle: nodes are PFSP_NODE50_DTYPE, evaluate only."""
+    20 jobs (ta031..ta060) create a MAX_JOBS = 50 handle: nodes are PFSP_NODE50_DTYPE, for every entry point."""
 
     def __init__(self, inst: int | None = None, tables=None, M: int = 50000, device: int = 0):
         if tables is None:
@@ -76,6 +81,11 @@ class PfspEvaluator:
     def unregister_host(self, arr: np.ndarray) -> None:
         check(lib().tsb_pfsp_unregister_host(self._h, arr.ctypes.data), "tsb_pfsp_unregister_host")
 
+    def _nodes(self, nodes: np.ndarray, where: str) -> None:
+        """a node array of this handle's build (88-byte records, or 208-byte ones on a MAX_JOBS = 50 handle)"""
+        if nodes.dtype != self.node_dtype or not nodes.flags.c_contiguous:
+            raise TsbError(EINVAL, f"{where}: nodes must be a C-contiguous {self.node_dtype.itemsize}-byte node array")
+
     @property
     def kernel_launches(self) -> int:
         return int(lib().tsb_pfsp_kernel_launches(self._h))
@@ -108,17 +118,17 @@ class PfspEvaluator:
     def expand(self, parents: np.ndarray, lb, best: int):
         """(children, n_solutions, best_after): evaluate_gpu (pfsp_gpu_chpl.chpl:192-270) + generate_children
         (:273-303) of one chunk in one device pass"""
-        assert parents.dtype == PFSP_NODE_DTYPE and parents.flags.c_contiguous
+        self._nodes(parents, "tsb_pfsp_expand")
         kind = LB_NAMES[lb] if isinstance(lb, str) else int(lb)
         cap = parents.shape[0] * self.jobs
-        out = np.empty(max(cap, 1), dtype=PFSP_NODE_DTYPE)
+        out = np.empty(max(cap, 1), dtype=self.node_dtype)
         nc, ns, b = C.c_uint64(0), C.c_uint64(0), C.c_int64(int(best))
         check(lib().tsb_pfsp_expand(self._h, kind, parents.ctypes.data, parents.shape[0], C.byref(b), out.ctypes.data,
                                     cap, C.byref(nc), C.byref(ns)), "tsb_pfsp_expand")
         return out[: nc.value].copy(), int(ns.value), int(b.value)
 
     def pool_push(self, nodes: np.ndarray) -> None:
-        assert nodes.dtype == PFSP_NODE_DTYPE and nodes.flags.c_contiguous
+        self._nodes(nodes, "tsb_pfsp_pool_push")
         check(lib().tsb_pfsp_pool_push(self._h, nodes.ctypes.data, nodes.shape[0]), "tsb_pfsp_pool_push")
 
     @property
@@ -152,25 +162,33 @@ class PfspEvaluator:
 
     def pool_drain(self) -> np.ndarray:
         n = self.pool_size
-        out = np.empty(max(n, 1), dtype=PFSP_NODE_DTYPE)
+        out = np.empty(max(n, 1), dtype=self.node_dtype)
         got = C.c_int64(0)
         check(lib().tsb_pfsp_pool_drain(self._h, out.ctypes.data, n, C.byref(got)), "tsb_pfsp_pool_drain")
         return out[: got.value].copy()
 
 
 def pfsp_search_device(inst: int = 14, lb="lb1", ub: int = 1, m: int = 25, M: int = 50000, D: int = 1) -> SearchStats:
-    """same search, the pool(s) of step 2 resident on the device(s) (tsb_pfsp_pool_*)"""
+    """same search, the pool(s) of step 2 resident on the device(s) (tsb_pfsp_pool_*); ta031..ta060 run as the
+    MAX_JOBS = 50 build does"""
     kind = LB_NAMES[lb] if isinstance(lb, str) else int(lb)
     st = SearchStats()
-    check(lib().tsb_pfsp_search_device(inst, kind, ub, m, M, D, C.byref(st)), "tsb_pfsp_search_device")
+    if _max_jobs(inst) == 50:
+        check(lib().tsb_pfsp_search_device_wide(50, inst, kind, ub, m, M, D, C.byref(st)), "tsb_pfsp_search_device_wide")
+    else:
+        check(lib().tsb_pfsp_search_device(inst, kind, ub, m, M, D, C.byref(st)), "tsb_pfsp_search_device")
     return st
 
 
 def pfsp_search(inst: int = 14, lb="lb1", ub: int = 1, m: int = 25, M: int = 50000, D: int = 1) -> SearchStats:
-    """pfsp_gpu_chpl.chpl:306-431 (D = 1) / pfsp_multigpu_chpl.chpl (static split), C++ emulation driver"""
+    """pfsp_gpu_chpl.chpl:306-431 (D = 1) / pfsp_multigpu_chpl.chpl (static split), C++ emulation driver; ta031..ta060
+    run as the MAX_JOBS = 50 build does"""
     kind = LB_NAMES[lb] if isinstance(lb, str) else int(lb)
     st = SearchStats()
-    check(lib().tsb_pfsp_search(inst, kind, ub, m, M, D, C.byref(st)), "tsb_pfsp_search")
+    if _max_jobs(inst) == 50:
+        check(lib().tsb_pfsp_search_wide(50, inst, kind, ub, m, M, D, C.byref(st)), "tsb_pfsp_search_wide")
+    else:
+        check(lib().tsb_pfsp_search(inst, kind, ub, m, M, D, C.byref(st)), "tsb_pfsp_search")
     return st
 
 

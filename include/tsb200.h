@@ -195,9 +195,10 @@ int tsb_pfsp_create(tsb_pfsp** h, int device, int jobs, int machines, int M_max,
                     const int32_t* johnson, const int32_t* lags, const int32_t* mp0, const int32_t* mp1,
                     const int32_t* mp_order);
 /* SURVEY §8(f4): the reference built with MAX_JOBS = max_jobs.  max_jobs == 20: tsb_pfsp_create.  max_jobs == 50:
- * nodes are 208-byte tsb_pfsp_node50 records, jobs must be 50 (ta031..ta060), bounds[p*50 + k]; tsb_pfsp_evaluate /
- * tsb_pfsp_evaluate_device work on such a handle (general kernels, csrc/pfsp_wide.cuh), the fused expand / pool
- * entry points return TSB_EUNSUPPORTED.  Table layouts as for tsb_pfsp_create with jobs = 50. */
+ * nodes are 208-byte tsb_pfsp_node50 records, jobs must be 50 (ta031..ta060), bounds[p*50 + k].  Every PFSP entry
+ * point below works on such a handle with 208-byte records in place of 88-byte ones: evaluate / evaluate_device
+ * (general kernels, csrc/pfsp_wide.cuh), the fused expand and the device pool (csrc/pfsp_wide_expand.cuh).
+ * Table layouts as for tsb_pfsp_create with jobs = 50. */
 int tsb_pfsp_create_wide(tsb_pfsp** h, int device, int max_jobs, int jobs, int machines, int M_max, const int32_t* p_times,
                          const int32_t* min_heads, const int32_t* min_tails, int nb_pairs, const int32_t* johnson,
                          const int32_t* lags, const int32_t* mp0, const int32_t* mp1, const int32_t* mp_order);
@@ -218,7 +219,9 @@ int tsb_pfsp_evaluate_device(tsb_pfsp* h, int lb_kind, const void* parents_d, in
  * chunk.  *best is the incumbent: read at entry, lowered to the smallest leaf bound of the chunk exactly as
  * the reference's sequential generate_children does (a round in which a leaf improves *best is redone through
  * the evaluate entry point and the sequential rule, so the children are the reference's in every case).
- * *n_solutions = evaluated leaf children (:283-288).  children come back packed, reference order. */
+ * *n_solutions = evaluated leaf children (:283-288).  children come back packed, reference order.  Nodes are the
+ * handle's records: 88-byte tsb_pfsp_node, or 208-byte tsb_pfsp_node50 on a MAX_JOBS = 50 handle; there
+ * children_d must be 16-byte aligned as well (TSB_EALIGN otherwise). */
 int tsb_pfsp_expand(tsb_pfsp* h, int lb_kind, const void* parents, int count, int64_t* best, void* children,
                     uint64_t capacity_nodes, uint64_t* n_children, uint64_t* n_solutions);
 int tsb_pfsp_expand_device(tsb_pfsp* h, int lb_kind, const void* parents_d /*16-B aligned*/, int count,
@@ -226,7 +229,10 @@ int tsb_pfsp_expand_device(tsb_pfsp* h, int lb_kind, const void* parents_d /*16-
                            uint64_t* n_solutions, void* stream);
 /* ---- device-resident pool (SURVEY §8f row 3), the PFSP twin of tsb_nq_pool_*: one offload round of
  * pfsp_gpu_chpl.chpl:376-392 (popBackBulk, evaluate, generate_children) per tsb_pfsp_pool_step, the pool kept
- * in HBM and read in place */
+ * in HBM and read in place.  Both builds (88- or 208-byte records, as the handle was created).  The arena starts
+ * at 4 * M_max * jobs nodes (at least 2^20; env TSB200_POOL_CAP overrides) and a second arena of the same size is
+ * allocated on the first compaction: on a MAX_JOBS = 50 handle with M_max = 50 000 that is 10 M x 208 B = 2.1 GB
+ * per arena.  tsb_pfsp_pool_steal moves nodes between two handles of the same build only (TSB_EINVAL otherwise). */
 int tsb_pfsp_pool_push(tsb_pfsp* h, const void* nodes, int64_t n);
 int64_t tsb_pfsp_pool_size(const tsb_pfsp* h);
 int tsb_pfsp_pool_step(tsb_pfsp* h, int lb_kind, int m, int M, int64_t* best, int64_t* n_parents,
@@ -313,15 +319,25 @@ int tsb_nq_search_on(tsb_nq* h, int N, int m, int M, tsb_search_stats* out);
 /* one task of that D-way split, on `device` — for process-per-GPU launches (one rank = one part): step 1 is
  * credited to part 0 and each part drains its own leftovers, so the parts' counts add up to the whole search */
 int tsb_nq_search_device_part(int N, int g, int m, int M, int D, int part, int device, tsb_search_stats* out);
-/* pfsp_gpu_chpl.chpl:306-431 / pfsp_multigpu_chpl.chpl:316-560 */
+/* pfsp_gpu_chpl.chpl:306-431 / pfsp_multigpu_chpl.chpl:316-560, as the MAX_JOBS = 20 build runs them (jobs <= 20:
+ * ta001..ta030; TSB_EUNSUPPORTED for larger instances) */
 int tsb_pfsp_search(int inst, int lb_kind, int ub, int m, int M, int D, tsb_search_stats* out);
 /* the same with the pool(s) of step 2 resident on the device(s) (tsb_pfsp_pool_*) */
 int tsb_pfsp_search_device(int inst, int lb_kind, int ub, int m, int M, int D, tsb_search_stats* out);
+/* the two searches as the reference built with MAX_JOBS = max_jobs runs them (`chpl -sMAX_JOBS=50`,
+ * lib/pfsp/PFSP_node.chpl:7): max_jobs == 20 is tsb_pfsp_search / tsb_pfsp_search_device; max_jobs == 50 takes
+ * ta031..ta060 with 208-byte nodes (TSB_EUNSUPPORTED for any other instance); any other max_jobs is
+ * TSB_EUNSUPPORTED.  Arguments are checked before any device is touched.  D > 1 as for 20 jobs: static split,
+ * device pools that steal from each other under ub = 1. */
+int tsb_pfsp_search_wide(int max_jobs, int inst, int lb_kind, int ub, int m, int M, int D, tsb_search_stats* out);
+int tsb_pfsp_search_device_wide(int max_jobs, int inst, int lb_kind, int ub, int m, int M, int D,
+                                tsb_search_stats* out);
 /* one task of the split (see tsb_nq_search_device_part).  The parts do not exchange their incumbent: with ub = 1 (the
  * optimum is known up front) the parts' counts add up to the whole search's; with ub = 0 every part prunes with the
  * best it finds itself, so the sum of the parts can exceed the single-process count (the optimum is still found). */
 int tsb_pfsp_search_device_part(int inst, int lb_kind, int ub, int m, int M, int D, int part, int device,
                                 tsb_search_stats* out);
+/* the D = 1 device-pool search on a handle the caller created; a MAX_JOBS = 50 handle runs ta031..ta060 */
 int tsb_pfsp_search_on(tsb_pfsp* h, int inst, int lb_kind, int ub, int m, int M, tsb_search_stats* out);
 
 #ifdef __cplusplus
